@@ -552,6 +552,13 @@ def workload_name(w):
             f"{w['samples_per_piece']} samples/piece, mesh-SDF robot ({w['mesh']}), discrete collision cost+grad")
 
 
+def dump_outputs(out_dir, **arrays):
+    """--dump-outputs: one float64 .npy per array, so that two builds run with the same arguments can be compared output for output"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 # ---- GPU arm ----------------------------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch
@@ -654,6 +661,7 @@ def run_ours(args):
     barrier()
     wall = time.perf_counter() - t_wall0
     launches = ev.stats().kernel_launches - l0
+    last = d_out.cpu().numpy().copy()                       # [cost | gradC | gradT] of the last timed step (--dump-outputs)
     k_last = n_warm + args.steps - 1
     # context figures (not the headline): warm L2; the SAME iterate repeated (round 1's measurement: the schedule is a perfect predictor);
     # cold = a context's first evaluation (natural sample order, nothing split)
@@ -803,6 +811,8 @@ def run_ours(args):
                                 "error seen through the hinge, reported as SURVEY 8c demands — not a parity claim"}
             except Exception as e:
                 line["extra"]["sign_policy_deviation_vs_reference_fwn"] = {"error": repr(e)}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, cost=last[:1], gradC=last[1:1 + 18 * N], gradT=last[1 + 18 * N:])
         print(json.dumps(line))
     if world > 1:
         import torch.distributed as dist
@@ -1156,7 +1166,13 @@ def main():
                     help="discrete = BASELINE configs[2] (headline); swept = configs[3]; batch1024 = configs[4] — each a strong-scaling workload of its own")
     ap.add_argument("--batch-total", type=int, default=1024, help="--workload batch1024: total problems (sharded over the ranks)")
     ap.add_argument("--lbfgs-iterations", type=int, default=8, help="--workload batch1024: iteration cap of the device-resident L-BFGS measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write cost, gradC and gradT of the last timed step as DIR/<name>.npy "
+                                                           "(float64; default discrete workload only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "discrete"):
+        ap.error("--dump-outputs applies to the default discrete workload of --impl ours")
     if args.impl == "reference":
         return run_reference(args) if args.workload == "discrete" else run_reference_other(args)
     if args.workload == "swept":

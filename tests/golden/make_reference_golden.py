@@ -8,7 +8,10 @@ Run in the build container (where /root/reference exists):  python tests/golden/
   minco_reference.npz — outputs of the reference's utils/minco.hpp (MINCO_S3NU forward, energy gradients, propogateGrad) on seeded problems, and
                         of its utils/trajectory.hpp (getPos_Vel_Acc_Jerk, locatePieceIdx, getTotalDuration) on the resulting trajectories;
   lbfgs_reference.npz — what the reference's utils/lbfgs.hpp does on seeded problems: every evaluated point, solution, value, return code;
-  grid_reference.npz  — the reference's map_manager/src/Gridmap3D.cpp: grid indices, cube centres, in-map flags and AABB gathers on seeded grids."""
+  grid_reference.npz  — the reference's map_manager/src/Gridmap3D.cpp: grid indices, cube centres, in-map flags and AABB gathers on seeded grids;
+  reference_pins.npz  — what the tests that call the reference-compiled libraries compare against, for where oracle/_ref is absent: the
+                        reference's OBJ files as shipped (bytes), flatness.hpp on a fixed sample of the 10000 random inputs, FWN winding
+                        numbers, the FWN-signed oracle (s = 1 - 2 w) on the robot meshes and on the sign-policy cases, getTrajectory."""
 import os
 import sys
 import numpy as np
@@ -19,7 +22,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "implicit-sdf-planner_b200", "py"))
 import isdf_b200 as I          # noqa: E402
 import oracle_lib as O         # noqa: E402
-from test_reference_pins import flat_inputs, _minco_cases, _lbfgs_problems, _traj_times, _grid_cases   # noqa: E402
+from test_reference_pins import flat_inputs, _minco_cases, _lbfgs_problems, _traj_times, _grid_cases, N_RANDOM, FLAT_SAMPLE   # noqa: E402
 
 
 REF_SHAPES = "/root/reference/src/plan_manager/shapes"
@@ -45,6 +48,36 @@ def ref_meshes():
         print(name, V.shape, F.shape, "w range", w.min(), w.max())
     np.savez_compressed(os.path.join(HERE, "ref_meshes.npz"), names=np.array(list(MESHES)), **out)
     print("ref_meshes.npz written")
+
+
+def reference_pins():
+    from common import MESHES as TEST_MESHES
+    from test_oracle_pins import fwn_kat_points
+    from test_gpu_reference_pins import sign_policy_case
+    out = {}
+    for name in MESHES:
+        out["obj_" + name] = np.frombuffer(open(os.path.join(REF_SHAPES, name + ".obj"), "rb").read(), dtype=np.uint8)
+    cfg = O.config_from(I.default_config_values())
+    ref = O.RefFlat(cfg)
+    v, a, j, pg, vg, qg, og = (x[FLAT_SAMPLE] for x in flat_inputs(N_RANDOM))
+    out["flat_quat"], out["flat_omg"] = ref.forward(v, a, j)
+    out["flat_quat_only"] = ref.forward_quat(v, a, j)
+    out["flat_back"] = ref.backward(v, a, j, pg, vg, qg, og)
+    for name, gen in TEST_MESHES.items():
+        V, F = gen()
+        out[f"fwn_{name}_w"] = O.RefFwn(V, F, order=2).query(fwn_kat_points(), 2.0)
+    z = np.load(os.path.join(HERE, "ref_meshes.npz"))
+    for name in MESHES:
+        V, F, pp, q = z[name + "_V"], z[name + "_F"], z[name + "_pp"], z[name + "_q"]
+        out[f"mesh_{name}_sdf_fwn"], out[f"mesh_{name}_grad_fwn"] = O.Shape.mesh(V, F, pp, wn_mode=O.WN_REF).query(q)
+    for name in ("Lthick", "RoundedCone"):
+        cfg_s, occ, T, Cc, V, F, pp = sign_policy_case(name)
+        out[f"sign_{name}_cost"], out[f"sign_{name}_gradC"], out[f"sign_{name}_gradT"], _ = O.eval_discrete(
+            O.config_from(cfg_s), occ, [0, 0, 0], 1.0, O.Shape.mesh(V, F, pp, wn_mode=O.WN_REF), T, Cc)
+    N, head, tail, inPs, T, _, _ = _minco_cases()[2]
+    out["traj_durations"], out["traj_coeffs"] = O.RefMinco().trajectory(head, tail, inPs, T)
+    np.savez_compressed(os.path.join(HERE, "reference_pins.npz"), **out)
+    print("reference_pins.npz written")
 
 
 def main():
@@ -86,6 +119,7 @@ def main():
             out.update({f"g{k}_b{b}_pts": p_, f"g{k}_b{b}_n": np.array(n_)})
     np.savez_compressed(os.path.join(HERE, "grid_reference.npz"), **out)
     print("grid_reference.npz written")
+    reference_pins()
 
 
 if __name__ == "__main__":

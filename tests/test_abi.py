@@ -32,6 +32,7 @@ def test_library_exports_every_declared_symbol():
 
 def test_no_torch_or_oracle_linked_into_product():
     out = subprocess.check_output(["ldd", I.LIB_PATH]).decode()
+    out = re.sub(r"\(0x[0-9a-f]+\)", "", out)            # load addresses are random hex and can spell "c10"
     assert "torch" not in out and "oracle" not in out and "c10" not in out
     # the product sources never include the oracle
     for dirpath, _, files in os.walk(os.path.join(ROOT, "implicit-sdf-planner_b200")):
