@@ -3,6 +3,7 @@
 #include "../../include/isdf.h"
 #include "isdf_types.cuh"
 #include "isdf_discrete.cuh"
+#include "isdf_check.cuh"
 #include "isdf_swept.cuh"
 #include "isdf_minco.cuh"
 #include "isdf_frontend.cuh"
@@ -89,6 +90,9 @@ struct isdf_ctx {
     bool peer_fused = false;             // sharded *_device evaluations finish with the exchange
     int peer_world_alloc = 0, peer_cap = 0;
     DevBuf<int> d_peer_status;
+    // collision check (isdf_check.cuh): its own buffers, so that a check leaves the cost paths' state alone
+    DevBuf<double> d_ck_in, d_ck_clear; DevBuf<long long> d_ck_arg; DevBuf<int> d_ck_cursor; DevBuf<unsigned long long> d_ck_counters, d_ck_cycles;
+    DevBuf<isdf_clearance_report> d_ck_rep;
     isdf_stats stats;
 };
 
@@ -182,6 +186,7 @@ extern "C" int isdf_destroy(isdf_ctx *c) {
     c->d_fe_rot.release(); c->d_fe_kernels.release(); c->d_fe_order.release(); c->d_fe_ok.release(); c->d_fe_masks.release(); c->d_fe_out.release(); c->d_fe_ind.release(); c->d_fe_father.release(); c->d_fe_child.release(); c->d_fe_core.release(); c->d_fe_urows.release(); c->d_fe_surv.release(); c->d_fe_chunks.release(); c->d_fe_tab.release(); c->d_fe_count.release();
     c->d_mx.release(); c->d_mbc.release(); c->d_mT.release(); c->d_mC.release(); c->d_mlu.release(); c->d_men.release(); c->d_mgC.release(); c->d_mgT.release(); c->d_mcost.release(); c->d_mgrad.release(); c->d_mout.release(); c->d_mCpp.release(); c->d_msv.release();
     c->sv.release();
+    c->d_ck_in.release(); c->d_ck_clear.release(); c->d_ck_arg.release(); c->d_ck_cursor.release(); c->d_ck_counters.release(); c->d_ck_cycles.release(); c->d_ck_rep.release();
     if (c->h_stage) cudaFreeHost(c->h_stage);
     if (c->h_lb_active) cudaFreeHost(c->h_lb_active);
     c->d_lb_x.release(); c->d_lb_f.release(); c->d_lb_grad.release(); c->d_lb_state.release(); c->d_lb_int.release(); c->d_lb_head.release();
@@ -1465,6 +1470,109 @@ extern "C" int isdf_get_swept_results(isdf_ctx *c, double *tstar, double *sdf, d
 }
 
 
+// ---- whole-body collision check (isdf_check.cuh) ------------------------------------------------------------------
+static void poison_reports(isdf_clearance_report *r, int B) {
+    if (!r || B < 1) return;
+    const double nan = std::numeric_limits<double>::quiet_NaN();
+    for (int b = 0; b < B; b++) {
+        isdf_clearance_report &x = r[b];
+        x.min_clearance = x.t_min = x.t_hit = nan;
+        for (int a = 0; a < 3; a++) x.p_min[a] = x.p_hit[a] = nan;
+        x.collides = 1; x.piece_min = x.sample_min = x.piece_hit = x.sample_hit = -1; x.reserved_ = 0;
+    }
+}
+
+static int check_args(isdf_ctx *c, int B, int N0, int M, double margin, double horizon) {
+    if (B < 1 || N0 < 1) return fail(ISDF_ERR_INVALID, "B and N0 must be >= 1");
+    if (M < 1 || M > CHECK_MAX_SAMPLES_PER_PIECE) return fail(ISDF_ERR_INVALID, "samples_per_piece must be in [1, 4096]");
+    if ((long long)B * N0 > 0x7fffffffll || (long long)B * N0 * (M + 1) > 0x7fffffffll) return fail(ISDF_ERR_INVALID, "B * N0 * (samples_per_piece + 1) must fit in 31 bits");
+    if (!std::isfinite(horizon) || !(horizon > 0.0)) return fail(ISDF_ERR_INVALID, "horizon must be finite and > 0");
+    if (!std::isfinite(margin) || margin > horizon) return fail(ISDF_ERR_INVALID, "margin must be finite and <= horizon");
+    if (!c) return fail(ISDF_ERR_INVALID, "ctx is NULL");
+    if (!c->have_map) return fail(ISDF_ERR_STATE, "map not set");
+    if (!c->have_shape) return fail(ISDF_ERR_STATE, "shape not set");
+    return 0;
+}
+
+// both entry points: per-sample kernel + per-trajectory finisher on st (asynchronous)
+static int check_launch_ctx(isdf_ctx *c, int B, int N0, const double *d_T, const double *d_C, int M, double margin, double horizon,
+                            isdf_clearance_report *d_rep, double *d_clear, cudaStream_t st) {
+    const int N = B * N0;
+    const size_t S = (size_t)N * (M + 1);
+    if (c->d_ck_cursor.n < 1) {
+        CU_TRY(c->d_ck_cursor.ensure(1));
+        CU_TRY(cudaMemsetAsync(c->d_ck_cursor.p, 0, sizeof(int), st));
+    }
+    CU_TRY(c->d_ck_arg.ensure(S));
+    if (!d_clear) { CU_TRY(c->d_ck_clear.ensure(S)); d_clear = c->d_ck_clear.p; }
+    CU_TRY(c->d_ck_counters.ensure(CHECK_NCOUNTERS));
+    CU_TRY(cudaMemsetAsync(c->d_ck_counters.p, 0, sizeof(unsigned long long) * CHECK_NCOUNTERS, st));
+    CheckArgs A;
+    A.cfg = c->dcfg; A.grid = c->grid; A.shape = c->shape;
+    A.N = N; A.N0 = N0; A.M = M; A.T = d_T; A.C = d_C; A.margin = margin; A.horizon = horizon;
+    A.clear = d_clear; A.arg = c->d_ck_arg.p; A.cursor = c->d_ck_cursor.p; A.counters = c->d_ck_counters.p; A.reports = d_rep;
+    A.cycles = nullptr;
+    if (c->dbg_on) { CU_TRY(c->d_ck_cycles.ensure(S)); A.cycles = c->d_ck_cycles.p; }
+    const int mode = c->shape.kind != ISDF_SHAPE_MESH ? CHECK_ANALYTIC : (c->shape.mesh.sign_mode == MESH_SIGN_WINDING ? CHECK_MESH_WINDING : CHECK_MESH_EXACT);
+    CU_TRY(check_launch(A, mode, B, c->sm_count, st));
+    c->stats.kernel_launches += 2;
+    return 0;
+}
+
+extern "C" int isdf_check_collision(isdf_ctx *c, int B, int N0, const double *T, const double *coeffs, int samples_per_piece,
+                                    double margin, double horizon, isdf_clearance_report *reports, double *clearance) {
+    poison_reports(reports, B);
+    int r = check_args(c, B, N0, samples_per_piece, margin, horizon);
+    if (r) return r;
+    if (!T || !coeffs || !reports) return fail(ISDF_ERR_INVALID, "NULL argument");
+    auto body = [&]() -> int {
+        if (set_device(c)) return ISDF_ERR_CUDA;
+        const int N = B * N0;
+        const size_t S = (size_t)N * (samples_per_piece + 1);
+        // [coefficients 18N | durations N] in one copy
+        CU_TRY(c->d_ck_in.ensure((size_t)19 * N));
+        CU_TRY(cudaMemcpyAsync(c->d_ck_in.p, coeffs, sizeof(double) * 18 * N, cudaMemcpyHostToDevice, c->stream));
+        CU_TRY(cudaMemcpyAsync(c->d_ck_in.p + 18 * (size_t)N, T, sizeof(double) * N, cudaMemcpyHostToDevice, c->stream));
+        CU_TRY(c->d_ck_rep.ensure(B));
+        int rr = check_launch_ctx(c, B, N0, c->d_ck_in.p + 18 * (size_t)N, c->d_ck_in.p, samples_per_piece, margin, horizon, c->d_ck_rep.p,
+                                  nullptr, c->stream);
+        if (rr) return rr;
+        std::vector<isdf_clearance_report> tmp(B);
+        CU_TRY(cudaMemcpyAsync(tmp.data(), c->d_ck_rep.p, sizeof(isdf_clearance_report) * B, cudaMemcpyDeviceToHost, c->stream));
+        if (clearance) CU_TRY(cudaMemcpyAsync(clearance, c->d_ck_clear.p, sizeof(double) * S, cudaMemcpyDeviceToHost, c->stream));
+        CU_TRY(cudaStreamSynchronize(c->stream));
+        std::memcpy(reports, tmp.data(), sizeof(isdf_clearance_report) * B);
+        return 0;
+    };
+    r = body();
+    if (r) poison_reports(reports, B);
+    return r;
+}
+
+extern "C" int isdf_check_collision_device(isdf_ctx *c, int B, int N0, const double *d_T, const double *d_coeffs, int samples_per_piece,
+                                           double margin, double horizon, isdf_clearance_report *d_reports, double *d_clearance,
+                                           void *cuda_stream) {
+    const cudaStream_t st = (cudaStream_t)cuda_stream;
+    auto poison_dev = [&]() {   // the device reports read "not safe" on every failure (best effort: the launch itself may be what failed)
+        if (!d_reports || B < 1) return;
+        int dev = -1;
+        if (c) dev = c->device;
+        else {
+            cudaPointerAttributes pa;
+            if (cudaPointerGetAttributes(&pa, d_reports) != cudaSuccess || pa.type != cudaMemoryTypeDevice) { cudaGetLastError(); return; }
+            dev = pa.device;
+        }
+        if (cudaSetDevice(dev) == cudaSuccess) check_launch_poison(d_reports, B, st);
+        cudaGetLastError();
+    };
+    int r = check_args(c, B, N0, samples_per_piece, margin, horizon);
+    if (!r && (!d_T || !d_coeffs || !d_reports)) r = fail(ISDF_ERR_INVALID, "NULL device pointer");
+    if (!r && set_device(c)) r = ISDF_ERR_CUDA;
+    if (!r) r = check_launch_ctx(c, B, N0, d_T, d_coeffs, samples_per_piece, margin, horizon, d_reports, d_clearance, st);
+    if (r) poison_dev();
+    return r;
+}
+
 // ---- internal diagnostics (not part of include/isdf.h) ------------------------------------------------------------
 extern "C" int isdf_dbg_enable(isdf_ctx *c, int on) { if (!c) return -1; c->dbg_on = on != 0; c->sv.dbg_on = on != 0; return 0; }
 // scheduling diagnostics: natural_order != 0 -> every launch in natural sample order, nothing split (the state of a context's FIRST
@@ -1519,4 +1627,14 @@ extern "C" int isdf_dbg_sample_stats(isdf_ctx *c, unsigned long long *out, long 
     if (!c || !out || (size_t)n > c->d_dbg.n) return -1;
     if (cudaSetDevice(c->device) != cudaSuccess) return -3;
     return cudaMemcpy(out, c->d_dbg.p, sizeof(unsigned long long) * n, cudaMemcpyDeviceToHost) == cudaSuccess ? 0 : -3;
+}
+// collision check diagnostics: counters {voxels in the body box, SDF values computed, mesh searches} of the last check and, after
+// isdf_dbg_enable(ctx, 1), the per-sample clock64 cycles of its warp (n = samples of that check; may be 0)
+extern "C" int isdf_dbg_check_stats(isdf_ctx *c, unsigned long long *counters3, unsigned long long *cycles, long long n) {
+    if (!c || !counters3 || !c->d_ck_counters.p || (n > 0 && (!cycles || (size_t)n > c->d_ck_cycles.n))) return -1;
+    if (cudaSetDevice(c->device) != cudaSuccess) return -3;
+    if (cudaStreamSynchronize(c->stream) != cudaSuccess) return -3;
+    if (cudaMemcpy(counters3, c->d_ck_counters.p, sizeof(unsigned long long) * CHECK_NCOUNTERS, cudaMemcpyDeviceToHost) != cudaSuccess) return -3;
+    if (n > 0 && cudaMemcpy(cycles, c->d_ck_cycles.p, sizeof(unsigned long long) * n, cudaMemcpyDeviceToHost) != cudaSuccess) return -3;
+    return 0;
 }

@@ -185,20 +185,24 @@ __device__ __forceinline__ void scan_window(const DevGrid &G, const Window &W, i
     }
 }
 
-// pose of sample (i, j): position, flatness quaternion, rotation (hpp:456-492)
-__device__ __forceinline__ void sample_pose(const DiscArgs &A, int i, int j, double step, d3 &pos, quat4 &q, rot3 &R) {
+// pose of piece i of the 6N x 3 column-major block C at local time j * step: position, flatness quaternion, rotation (hpp:456-492)
+__device__ __forceinline__ void piece_pose(const double *C, int N, int i, int j, double step, const FlatParams &fp, d3 &pos, quat4 &q, rot3 &R) {
     double cx[6], cy[6], cz[6];
 #pragma unroll
     for (int k = 0; k < 6; k++) {
-        cx[k] = __ldg(A.C + 6 * i + k);
-        cy[k] = __ldg(A.C + 6 * A.N + 6 * i + k);
-        cz[k] = __ldg(A.C + 12 * A.N + 6 * i + k);
+        cx[k] = __ldg(C + 6 * i + k);
+        cy[k] = __ldg(C + 6 * N + 6 * i + k);
+        cz[k] = __ldg(C + 12 * N + 6 * i + k);
     }
     PieceEval pe;
     piece_eval(cx, cy, cz, j * step, pe);
-    q = flat_quat_only(A.cfg.fp, pe.vel, pe.acc);
+    q = flat_quat_only(fp, pe.vel, pe.acc);
     pos = pe.pos;
     R = quat_rot(q);
+}
+// pose of sample (i, j)
+__device__ __forceinline__ void sample_pose(const DiscArgs &A, int i, int j, double step, d3 &pos, quat4 &q, rot3 &R) {
+    piece_pose(A.C, A.N, i, j, step, A.cfg.fp, pos, q, R);
 }
 
 // hpp:505-551 for one sample given the reduced collision sums; writes the 20 per-sample partials to st[]

@@ -1,5 +1,5 @@
 // Translation unit of the discrete-path kernels (isdf_discrete.cuh): k_discrete_mesh, k_discrete_analytic, k_discrete_epilogue,
-// k_build_items. Compiled WITH FMA contraction (nvcc default): nothing on this path replays a sequential decision of the
+// k_build_items, and the collision-check kernels (isdf_check.cuh: k_check_samples, k_check_finish). Compiled WITH FMA contraction (nvcc default): nothing on this path replays a sequential decision of the
 // reference, its parity bar is the north star's 1e-6 (observed ~1e-15), and un-fused FP64 cost the mesh kernel ~12 % (ncu,
 // profiles/r01_p). The swept-volume search, whose accept/reject sequence must replay the reference's bit for bit, stays in
 // isdf_api.cu under -fmad=false. ISDF_FAST_TRI selects the division-free closest-point test (isdf_mesh.cuh) for this TU only.
@@ -10,6 +10,8 @@
 #include "../../include/isdf.h"
 #include "isdf_types.cuh"
 #include "isdf_discrete.cuh"
+#include "isdf_check.cuh"
+#include <algorithm>
 
 namespace isdf {
 
@@ -71,6 +73,32 @@ __global__ void k_dbg_flatness(const FlatParams fp, int n, const double *vaj, co
 
 cudaError_t discrete_launch_dbg_flatness(const FlatParams &fp, int n, const double *vaj, const double *grads, double *out, cudaStream_t st) {
     k_dbg_flatness<<<(n + 127) / 128, 128, 0, st>>>(fp, n, vaj, grads, out);
+    return cudaGetLastError();
+}
+
+cudaError_t check_launch(const CheckArgs &A, int mode, int B, int sm_count, cudaStream_t st) {
+    static int resident[3] = {0, 0, 0};   // CTAs per SM of each sample kernel (occupancy API, asked once)
+    const void *fn = mode == CHECK_ANALYTIC ? (const void *)k_check_samples<CHECK_ANALYTIC>
+                   : mode == CHECK_MESH_EXACT ? (const void *)k_check_samples<CHECK_MESH_EXACT> : (const void *)k_check_samples<CHECK_MESH_WINDING>;
+    if (resident[mode] == 0) {
+        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&resident[mode], fn, CHECK_THREADS, 0);
+        if (e != cudaSuccess) return e;
+        resident[mode] = std::max(resident[mode], 1);
+    }
+    // persistent grid: one CTA per resident slot, or fewer when there are fewer samples than warps
+    const long long S = (long long)A.N * (A.M + 1);
+    const long long grid = std::max(1ll, std::min((S + CHECK_WARPS - 1) / CHECK_WARPS, (long long)sm_count * resident[mode]));
+    if (mode == CHECK_ANALYTIC) k_check_samples<CHECK_ANALYTIC><<<(unsigned)grid, CHECK_THREADS, 0, st>>>(A);
+    else if (mode == CHECK_MESH_EXACT) k_check_samples<CHECK_MESH_EXACT><<<(unsigned)grid, CHECK_THREADS, 0, st>>>(A);
+    else k_check_samples<CHECK_MESH_WINDING><<<(unsigned)grid, CHECK_THREADS, 0, st>>>(A);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    k_check_finish<<<(unsigned)B, CHECK_FIN_THREADS, 0, st>>>(A);
+    return cudaGetLastError();
+}
+
+cudaError_t check_launch_poison(isdf_clearance_report *d_reports, int B, cudaStream_t st) {
+    k_check_poison<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(d_reports, B);
     return cudaGetLastError();
 }
 

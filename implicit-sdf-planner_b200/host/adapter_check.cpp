@@ -42,6 +42,14 @@ void isdf_host_backend_last(void *be, double *cost_pos, double *cost_other, doub
     BackEnd *b = (BackEnd *)be;
     *cost_pos = b->cost_pos; *cost_other = b->cost_other; *cost_total = b->cost_total; *status = b->last_status;
 }
+// BackEnd::isTrajCollide on decision vector x (reports into *rep); returns 1 = collides or failed, 0 = collision-free
+int isdf_host_backend_collides(void *be, const double *x, int check_samples, double margin, double horizon, isdf_clearance_report *rep, int *status) {
+    BackEnd *b = (BackEnd *)be;
+    b->check_samples = check_samples;
+    const bool hit = b->isTrajCollide(x, margin, horizon, rep);
+    if (status) *status = b->last_status;
+    return hit ? 1 : 0;
+}
 void isdf_host_backend_destroy(void *be) { delete (BackEnd *)be; }
 void isdf_host_tau_maps(const double *tau, int n, double *T, double *tau_back) { BackEnd::forwardT(tau, T, n); BackEnd::backwardT(T, tau_back, n); }
 // OBJ reader (read_triangle_mesh counterpart): returns 0 and the counts; copies up to capV vertices / capF faces when the buffers are given

@@ -7,6 +7,8 @@
 //   addTimeIntPenaltyParallel) -> propogateGrad -> + rho * sum(T) -> backwardGradT / backwardGradP (hpp:283-330).
 // Both device calls ACCUMULATE into cost / gradT / gradC exactly like the reference's reference-arguments.
 // On a device error the cost is NaN (see include/isdf.h) so either optimiser driver stops.
+// BackEnd::isTrajCollide is the hard verdict the reference's SweptVolumeManager::isTrajCollide (sw_manager.hpp:759-767) only stubs:
+// the decision vector the optimiser returned -> the same trajectory costFunctionLmbm evaluates -> isdf_check_collision.
 #pragma once
 #include "isdf.h"
 #include "isdf_minco.hpp"
@@ -31,6 +33,7 @@ struct BackEnd {
     double cost_pos = 0, cost_other = 0, cost_total = 0;
     long cost_iter = 0;
     int last_status = 0;
+    int check_samples = 64;       // isTrajCollide: check intervals per piece (the natural choice: the context's integral_intervs)
 
     void setup(isdf_ctx *c, int pieces, const double *head3x3, const double *tail3x3) {
         ctx = c; N = pieces;
@@ -82,6 +85,21 @@ struct BackEnd {
         backwardGradT(x, o.gradTimes.data(), g, dimTau);
         for (int k = 0; k < dimXi; k++) g[dimTau + k] = o.gradPts[k];               // backwardGradP
         return cost;
+    }
+
+    // Does the trajectory of decision vector x (n = N + 3(N-1): what the optimiser returned) collide? Rebuilds the trajectory exactly
+    // as costFunctionLmbm does (forwardT, forwardP, MINCO) and checks it at check_samples + 1 samples per piece. Returns true on a hit
+    // AND on any error (rep->min_clearance is NaN then, last_status has the code): a failed check never reads "safe". rep may be NULL.
+    bool isTrajCollide(const double *x, double margin, double horizon, isdf_clearance_report *rep = nullptr) {
+        isdf_clearance_report local;
+        if (!rep) rep = &local;
+        const int dimTau = N, dimXi = 3 * (N - 1);
+        if (!ctx || N < 1 || !x) { last_status = ISDF_ERR_INVALID; rep->min_clearance = std::numeric_limits<double>::quiet_NaN(); rep->collides = 1; return true; }
+        forwardT(x, times.data(), dimTau);
+        for (int k = 0; k < dimXi; k++) points[k] = x[dimTau + k];
+        minco.setParameters(points.data(), times.data());
+        last_status = isdf_check_collision(ctx, 1, N, times.data(), minco.coeffs().data(), check_samples, margin, horizon, rep, nullptr);
+        return last_status != ISDF_OK || rep->collides != 0;
     }
 
     // raw twin of lbfgs_evaluate_t (the reference's fork adds the p_cost out-parameter, lbfgs.hpp:213-216)

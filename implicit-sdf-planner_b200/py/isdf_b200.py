@@ -31,7 +31,8 @@ ABI_SYMBOLS = ["isdf_default_config", "isdf_create", "isdf_destroy", "isdf_last_
                "isdf_gather_obstacle_points", "isdf_callback_batch", "isdf_callback_batch_device", "isdf_get_batch_trajectories",
                "isdf_lbfgs_default_params", "isdf_lbfgs_batch", "isdf_lbfgs_batch_device", "isdf_set_points_batch",
                "isdf_frontend_build_kernels", "isdf_frontend_get_kernels", "isdf_frontend_feasibility", "isdf_frontend_feasibility_device",
-               "isdf_frontend_check_batch", "isdf_peer_export", "isdf_peer_connect", "isdf_peer_allreduce_device", "isdf_peer_status", "isdf_peer_disconnect"]
+               "isdf_frontend_check_batch", "isdf_peer_export", "isdf_peer_connect", "isdf_peer_allreduce_device", "isdf_peer_status", "isdf_peer_disconnect",
+               "isdf_check_collision", "isdf_check_collision_device"]
 
 
 class KernelConfig(C.Structure):
@@ -56,6 +57,17 @@ class LbfgsParams(C.Structure):
     """isdf_lbfgs_params"""
     _fields_ = [(n, C.c_int32) for n in ["mem_size", "past", "max_iterations", "max_linesearch", "max_rounds", "reserved_"]] + \
                [(n, C.c_double) for n in ["g_epsilon", "delta", "min_step", "max_step", "f_dec_coeff", "cautious_factor", "machine_prec"]]
+
+
+class ClearanceReport(C.Structure):
+    """isdf_clearance_report — one per trajectory checked by isdf_check_collision (96 bytes)."""
+    _fields_ = [("min_clearance", C.c_double), ("t_min", C.c_double), ("p_min", C.c_double * 3), ("t_hit", C.c_double), ("p_hit", C.c_double * 3)] + \
+               [(n, C.c_int32) for n in ["collides", "piece_min", "sample_min", "piece_hit", "sample_hit", "reserved_"]]
+
+    def as_dict(self):
+        return dict(min_clearance=self.min_clearance, t_min=self.t_min, p_min=np.array(self.p_min[:]), t_hit=self.t_hit, p_hit=np.array(self.p_hit[:]),
+                    collides=bool(self.collides), piece_min=self.piece_min, sample_min=self.sample_min, piece_hit=self.piece_hit,
+                    sample_hit=self.sample_hit)
 
 
 class Stats(C.Structure):
@@ -126,6 +138,8 @@ def load_library(path=None):
     lib.isdf_peer_status.argtypes = [vp]
     lib.isdf_peer_disconnect.argtypes = [vp]
     lib.isdf_eval_swept_given.argtypes = [vp, C.c_int, dp, dp, dp, dp, dp, dp, dp, dp]
+    lib.isdf_check_collision.argtypes = [vp, C.c_int, C.c_int, dp, dp, C.c_int, C.c_double, C.c_double, C.POINTER(ClearanceReport), dp]
+    lib.isdf_check_collision_device.argtypes = [vp, C.c_int, C.c_int, vp, vp, C.c_int, C.c_double, C.c_double, vp, vp, vp]
     for s in ABI_SYMBOLS:
         if s != "isdf_last_error":
             getattr(lib, s).restype = C.c_int
@@ -300,6 +314,39 @@ class Evaluator:
         T, Cc, en = np.zeros(B * N0), np.zeros(18 * B * N0), np.zeros(B)
         self._check(self.lib.isdf_get_batch_trajectories(self.h, _dp(T), _dp(Cc), _dp(en)))
         return T, Cc, en
+
+    # ---- whole-body collision check (see include/isdf.h) ----
+    def check_collision(self, T, coeffs, samples_per_piece, margin, horizon, B=1, per_sample=False):
+        """B trajectories of N0 = len(T) / B pieces (coefficient block as eval_discrete / batch_trajectories) -> list of B report dicts,
+        plus the per-sample clearance (B, N0, M + 1) when per_sample. Raises IsdfError on failure (the library's reports are poisoned)."""
+        T = _f64(T).reshape(-1)
+        Cc = _f64(coeffs).reshape(-1)
+        assert T.size % B == 0 and Cc.size == 18 * T.size
+        N0, M = T.size // B, int(samples_per_piece)
+        reps = (ClearanceReport * B)()
+        clear = np.zeros(T.size * (M + 1)) if per_sample else None
+        self._check(self.lib.isdf_check_collision(self.h, B, N0, _dp(T), _dp(Cc), M, float(margin), float(horizon), reps, _dp(clear)))
+        out = [r.as_dict() for r in reps]
+        return (out, clear.reshape(B, N0, M + 1)) if per_sample else out
+
+    def check_collision_device(self, B, N0, d_T, d_coeffs, samples_per_piece, margin, horizon, d_reports, d_clearance=0, stream=0):
+        """device-resident twin: raw device pointers (d_reports: B * 96 bytes, d_clearance may be 0), asynchronous on `stream`"""
+        self._check(self.lib.isdf_check_collision_device(self.h, B, N0, C.c_void_p(d_T), C.c_void_p(d_coeffs), int(samples_per_piece), float(margin),
+                                                         float(horizon), C.c_void_p(d_reports), C.c_void_p(d_clearance or None), C.c_void_p(stream)))
+
+    def dbg_check_stats(self, n_samples=0):
+        """counters of the last check {voxels in the body box, SDF values, mesh searches} and (after dbg_enable) per-sample cycles"""
+        cnt = (C.c_ulonglong * 3)()
+        cyc = np.zeros(n_samples, dtype=np.uint64)
+        self.lib.isdf_dbg_check_stats.argtypes = [C.c_void_p, C.POINTER(C.c_ulonglong), C.c_void_p, C.c_longlong]
+        if self.lib.isdf_dbg_check_stats(self.h, cnt, cyc.ctypes.data if n_samples else None, n_samples) != 0:
+            raise IsdfError(-1, "isdf_dbg_check_stats failed")
+        return dict(voxels_in_box=cnt[0], sdf_values=cnt[1], mesh_searches=cnt[2]), cyc
+
+    def dbg_enable(self, on=True):
+        self.lib.isdf_dbg_enable.argtypes = [C.c_void_p, C.c_int]
+        if self.lib.isdf_dbg_enable(self.h, int(on)) != 0:
+            raise IsdfError(-1, "isdf_dbg_enable failed")
 
     # ---- front end: attitude kernels (see include/isdf.h) ----
     def frontend_build_kernels(self, max_roll=45.0, max_pitch=45.0, ang_res=9.0, front_end_safeh=0.0):

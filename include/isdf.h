@@ -200,6 +200,46 @@ int isdf_lbfgs_batch_device(isdf_ctx *ctx, int B, int N0, const double *d_head, 
                             const isdf_lbfgs_params *params, double *d_x, double *d_f, int32_t *d_ret, int32_t *d_iterations, int32_t *d_evaluations,
                             int32_t *rounds, void *cuda_stream);
 
+/* ---- whole-body collision check: the verdict PlannerManager::generateTraj asks for after every optimisation
+ * (plan_manager.cpp:306, :383) and SweptVolumeManager::isTrajCollide (swm:759-767) leaves as a stub that always returns false.
+ * The cost terms above are soft (hinge penalties, zero beyond safety_hor, smoothed over mu) and an optimiser may stop with obstacles
+ * inside the robot; this is the hard answer.
+ *
+ * Check samples: piece i is checked at M + 1 local times j * (T_i * (1/M)), j = 0..M (M = samples_per_piece, the rule of the discrete
+ * path's integral nodes; M = integral_intervs is the natural choice). Pose as the discrete path: position from the piece polynomial,
+ * attitude R from the flatness quaternion.
+ * Clearance of a sample, H = horizon > 0, half_bd = kernel_size * occupancy_resolution / 2 (the body box of hpp:800):
+ *     c = min( H, min over occupied voxels v with |R^T (p_v - x)|_inf <= half_bd + H of sdf_robot(R^T (p_v - x)) )
+ * p_v = voxel centre (getGridCubeCenter). Voxels outside the map are free (no projInMap clamping: a geometric query, not a replay of
+ * the gather). sdf_robot = the SDF of the current shape: any analytic kind, a mesh with ISDF_MESH_SIGN_EXACT, or a mesh with
+ * ISDF_MESH_SIGN_WINDING (s = 1 - 2 w). For a 1-Lipschitz SDF (exact-sign mesh, Ball, Box) of a robot inside its kernel cube the box
+ * changes nothing: c = min(H, minimum over ALL occupied voxel centres).
+ * Verdict: the trajectory COLLIDES when some check sample has c < margin (margin <= H; a negative margin is a penetration tolerance).
+ * For a 1-Lipschitz SDF, margin = res * sqrt(3) / 2 means "no occupied voxel cube touches the robot at any check sample".
+ * A sample whose pose is not finite has c = NaN and counts as a hit. Nothing between check samples is certified.
+ * First hit = the smallest (piece, j) with c < margin. Argmin voxel: among equal SDF values the smallest linear address
+ * ix*Y*Z + iy*Z + iz; the reported minimum is the first sample in (piece, j) order that attains it.
+ * Results are independent of scheduling: bit-identical run to run, alone or inside a batch, host or device entry point. */
+typedef struct isdf_clearance_report {      /* one per trajectory */
+    double min_clearance, t_min;            /* smallest c over all check samples, and its trajectory time */
+    double p_min[3];                        /* the obstacle voxel centre that attains it (NaN if c == horizon) */
+    double t_hit, p_hit[3];                 /* first sample with c < margin and its argmin voxel (t_hit = -1, p_hit NaN if none) */
+    int32_t collides, piece_min, sample_min, piece_hit, sample_hit, reserved_;   /* pieces local to the trajectory; -1 = none */
+} isdf_clearance_report;
+/* B trajectories of N0 pieces concatenated like isdf_eval_discrete's restart batches (T: B*N0, coeffs 6*B*N0 x 3 col-major;
+ * isdf_get_batch_trajectories returns exactly this). 1 <= samples_per_piece <= 4096. reports: B. clearance (may be NULL):
+ * B*N0*(M+1) doubles, the per-sample c, piece-major. Needs the map and the shape; ignores isdf_set_shard (always the whole
+ * trajectory) and the ISDF_WITH_COLLISION flag. Touches no state of the cost paths (work-item schedule, lastTstar).
+ * ISDF_ERR_INVALID: bad B / N0 / M, horizon not finite and > 0, margin not finite or > horizon, NULL reports / T / coeffs.
+ * ISDF_ERR_STATE: map or shape not set. On ANY failure every report reads min_clearance = NaN, collides = 1 (when reports is
+ * given): a caller that ignores the status never reads "safe". */
+int isdf_check_collision(isdf_ctx *ctx, int B, int N0, const double *T, const double *coeffs, int samples_per_piece,
+                         double margin, double horizon, isdf_clearance_report *reports, double *clearance);
+/* device-resident variant: every pointer on ctx's device, asynchronous on cuda_stream (a cudaStream_t, NULL = default stream) */
+int isdf_check_collision_device(isdf_ctx *ctx, int B, int N0, const double *d_T, const double *d_coeffs, int samples_per_piece,
+                                double margin, double horizon, isdf_clearance_report *d_reports, double *d_clearance,
+                                void *cuda_stream);
+
 /* ---- multi-GPU reduction through NVLink / NVSwitch peer memory (optional; ncclAllReduce over the same 19N+1 doubles is the
  * library alternative). One process per GPU. Sequence on every rank:
  *   isdf_set_shard(ctx, rank, world); isdf_peer_export(ctx, world, max_doubles, h) -> all-gather the 64-byte handles ->
